@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (ours; N>1 via torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   (CPU PIL path, rank 0 only)
+    python bench.py ... --dump-outputs DIR      (also save what the last timed step computed, see dump_outputs)
 
 A "step" is one pass of the hot path over one batch of synthetic uint8 HWC images:
 policy ops -> HFlip -> ToTensor -> Normalize -> NCHW fp16, with the per-sample decisions
@@ -30,6 +31,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOADS = {
     # name: (H, W, per-GPU batch, policy fn name, tail kind, cutout)
@@ -243,6 +245,7 @@ def workload_string(name):
 class _Workload:
     """Device-resident buffers + the pre-bound launch of one workload on this rank."""
     NSETS = 4      # input/output sets rotate so that no step finds its data in the 126 MB L2
+    DUMP_BYTES = 60 * 10**6     # --dump-outputs: float32 images kept from the last step's output (stays under 64 MB)
 
     def __init__(self, name, seed, rank, world):
         import torch
@@ -285,6 +288,16 @@ class _Workload:
         barrier()
         return ev0.elapsed_time(ev1), t0, time.perf_counter()
 
+    def last_output(self, steps, warmup):
+        """(images, rows): float32 copy of what the last of `steps` timed steps after `warmup` wrote, and which rows of
+        the batch they are.  An output larger than DUMP_BYTES is represented by a fixed, seeded sample of its images."""
+        import numpy as np
+        import torch
+        out = self.outs[(warmup + steps - 1) % self.NSETS]
+        n = min(self.B, self.DUMP_BYTES // (out[0].numel() * 4 + 8))
+        rows = np.arange(self.B) if n == self.B else np.sort(np.random.default_rng(0).choice(self.B, n, replace=False))
+        return out[torch.from_numpy(rows).to(out.device)].float().cpu().numpy(), rows
+
     def roofline(self, ms_per_step):
         peak, peak_src = measured_peak()
         alg = self.in_bytes + self.out_bytes          # 3HW read + 6 out_h out_w written (= 9HW when no crop)
@@ -310,7 +323,7 @@ def measure_mixup(args, rank, world, barrier, max_over_ranks):
     tail = TailSpec.imagenet(0, torch.float16)
     xs = [torch.from_numpy(synth_batch(b, H, W, 4321 + rank + 17 * i)).cuda() for i in range(2)]
     y = torch.arange(rank * b, (rank + 1) * b, device="cuda")
-    steps = max(10, min(args.steps, 50))
+    steps = args.steps
     tim = {}
     # world > 1: the exchange is fused into the mix kernel (partners read over NVLink peer memory); FAA_MIXUP_A2A=1 or a
     # failing peer mapping selects the NCCL all-to-all route
@@ -501,6 +514,8 @@ def run_ours(args):
     launches0 = _lib.lib.faa_launch_count()
     ms_local, t0, t1 = wl.timed(args.steps, args.warmup, barrier)
     launches = int(_lib.lib.faa_launch_count() - launches0)
+    if args.dump_outputs and rank == 0:          # (before any later launch reuses the output buffers)
+        dump_outputs(args.dump_outputs, *wl.last_output(args.steps, args.warmup))
     # keep the GPU busy a little longer if the region was too short for a clock sample
     if t1 - t0 < 0.4:
         tb = time.perf_counter()
@@ -542,7 +557,7 @@ def run_ours(args):
     also = {}
     for name in ([] if args.no_also else [n for n in ("cifar32_b512", "effnetb4_380_b256") if n != args.workload]):
         w2 = _Workload(name, args.seed, rank, world)
-        k2 = max(args.steps, 300)
+        k2 = args.steps
         ms2, _, _ = w2.timed(k2, max(args.warmup, 5), barrier)
         ms2 = max_over_ranks([ms2])[0]
         also[name] = {"value": world * w2.B * k2 / (ms2 / 1e3), "unit": "images/s", "steps": k2, "ms_per_step": ms2 / k2,
@@ -608,6 +623,17 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, images, rows):
+    """What the timed path returned to its caller in its last step: ``out.npy`` (float32 [n, 3, out_h, out_w], the
+    fp16 NCHW output widened exactly) and ``out_rows.npy`` (float64 [n], the batch rows those images are).  Inputs,
+    seed and step indices depend only on the arguments, so two builds run with the same arguments can be compared
+    array for array."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "out.npy"), images.astype(np.float32))
+    np.save(os.path.join(out_dir, "out_rows.npy"), rows.astype(np.float64))
+
+
 def run_reference(args):
     """Reference arm: the reference's own CPU implementation of the path - its Augmentation /
     CutoutDefault classes from ``oracle/_ref`` (verbatim reference package; falls back to the oracle port
@@ -618,7 +644,7 @@ def run_reference(args):
     H, W, B, *_ = WORKLOADS[args.workload]
     cores = host_cores()
     workers = max(1, cores)
-    steps = max(1, args.steps)
+    steps = args.steps
     warm = max(1, args.warmup)
     v, dt, kind = cpu_throughput(args.workload, steps, warm, workers)
     line = {
@@ -647,7 +673,13 @@ def main():
     ap.add_argument("--seed", type=int, default=2024)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-also", action="store_true", help="skip the extra single-GPU configurations (CIFAR b512, 380x380 b256)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/*.npy (float32, at most 64 MB; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the outputs of --impl ours")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)

@@ -26,6 +26,6 @@ Pillow.  The oracle is therefore pinned against *outputs of the reference
 itself run in the build container* (Pillow 12.2.0, torchvision 0.26.0, numpy
 2.3.5, CPython 3.12): ``tests/golden/make_golden.py`` imports
 ``/root/reference`` and writes the fixtures under ``tests/golden/``; the
-``-m "not gpu"`` tests check both oracle layers against those fixtures, and,
-whenever ``/root/reference`` is present, against the live reference.
+``-m "not gpu"`` tests check both oracle layers against those fixtures; no
+test needs the reference itself.
 """

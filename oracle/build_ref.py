@@ -100,17 +100,13 @@ def build(force: bool = False) -> str | None:
 
 
 def import_ref():
-    """Import the vendored reference (``oracle/_ref``), or the live one when only that exists.
+    """Import the vendored reference (``oracle/_ref``, placed by ``build()``).  Never reads or copies
+    the reference checkout itself, so callers (bench.py, tests) write nothing into the tree.
     Returns (augmentations, archive, aug_mixup, data) modules of the reference, or None."""
-    root = None
-    if os.path.isdir(os.path.join(DST, "FastAutoAugment")):
-        root = DST
-    elif os.path.isdir(os.path.join(REF_ROOT, "FastAutoAugment")):
-        root = build() or None
-    if root is None:
+    if not os.path.isdir(os.path.join(DST, "FastAutoAugment")):
         return None
-    if root not in sys.path:
-        sys.path.insert(0, root)
+    if DST not in sys.path:
+        sys.path.insert(0, DST)
     import torch_six_shim
     torch_six_shim.install()
     from FastAutoAugment import augmentations, archive, aug_mixup, data

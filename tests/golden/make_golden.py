@@ -10,7 +10,8 @@ seeded synthetic inputs, and writes
 
     tests/golden/golden_ops.npz      per-op outputs (19 ops x levels x 3 input kinds, 32x32 + 24x40)
     tests/golden/golden_chain.npz    policy outputs + full CIFAR chain fp32 + mixup
-    tests/golden/golden_hashes.json  sha256 digests (incl. the SURVEY.md 8c table at 32 and 224)
+    tests/golden/golden_hashes.json  sha256 digests (incl. the SURVEY.md 8c table at 32 and 224, the inputs of
+                                     golden_chain.npz, whole-policy outputs and the Lighting chain)
 
 Environment that produced the committed files: Pillow 12.2.0, numpy 2.3.5,
 torch 2.11.0, torchvision 0.26.0, CPython 3.12.3.
@@ -30,6 +31,8 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF = "/root/reference"
+sys.path.insert(0, os.path.dirname(HERE))
+from helpers import GOLDEN_POLICY_BATCHES, LIVE_POLICY_RUNS, live_input, make_chain_inputs, sha_policy, synth_batch  # noqa: E402
 
 
 def import_reference():
@@ -132,19 +135,18 @@ def main():
     hashes["chained_seeds_0_63"] = chained
 
     # ---- (4) policy outputs on mixed inputs, batch-sequential RNG (num_workers=0 order)
+    # (the inputs are regenerated by the tests from their seeds, helpers.make_chain_inputs, and pinned by digest)
     chain = {}
-    rng = np.random.default_rng(77)
-    for pol, shape, n in (("fa_reduced_cifar10", (32, 32), 96), ("autoaug_policy", (32, 32), 96),
-                          ("fa_reduced_svhn", (32, 32), 48), ("arsaug_policy", (24, 40), 48),
-                          ("fa_resnet50_rimagenet", (56, 56), 48)):
+    inputs = make_chain_inputs()
+    hashes["chain_inputs"] = {k: sha(a) for k, a in inputs.items()}
+    for pol, shape, n in GOLDEN_POLICY_BATCHES:
         policies = getattr(archive, pol)()
-        batch = np.stack([synth(shape, i % 3, rng) for i in range(n)])
+        batch = inputs["policy_%s_in" % pol]
         A = data.Augmentation(policies)
         random.seed(5)
         np.random.seed(5)
         torch.manual_seed(5)
         out = np.stack([np.asarray(A(PIL.Image.fromarray(a))) for a in batch])
-        chain["policy_%s_in" % pol] = batch
         chain["policy_%s_out" % pol] = out
 
     # ---- (5) the exact CIFAR transform_train (data.py:39-44 + :92 + :112), fp32
@@ -154,13 +156,11 @@ def main():
                     T.Normalize(data._CIFAR_MEAN, data._CIFAR_STD)])
     tt.transforms.insert(0, data.Augmentation(policies))
     tt.transforms.append(data.CutoutDefault(16))
-    rng = np.random.default_rng(99)
-    batch = np.stack([synth((32, 32), i % 3, rng) for i in range(64)])
+    batch = inputs["cifar_chain_in"]
     random.seed(11)
     np.random.seed(11)
     torch.manual_seed(11)
     out = torch.stack([tt(PIL.Image.fromarray(a)) for a in batch]).numpy()
-    chain["cifar_chain_in"] = batch
     chain["cifar_chain_out_f32"] = out
     hashes["cifar_chain_sha"] = sha(out)
 
@@ -169,11 +169,39 @@ def main():
     np.random.seed(3)
     x = torch.from_numpy(out[:16].copy())
     y = torch.arange(16)
-    mixed, t1, t2, lam = aug_mixup.mixup(x, y, 0.2)
-    chain["mixup_in"] = out[:16]
-    chain["mixup_out"] = mixed.numpy()
+    mixed, t1, t2, lam = aug_mixup.mixup(x, y, 0.2)      # (its input is cifar_chain_out_f32[:16])
+    hashes["mixup_out"] = sha(mixed.numpy())
     chain["mixup_t2"] = t2.numpy()
     chain["mixup_lam"] = np.array([lam], dtype=np.float64)
+
+    # ---- (7) whole policies on fresh inputs, image by image (the reference's Augmentation loop, data.py:257-264);
+    #      16-hex-digit digests keep the fixture small, a mismatch still names the image
+    live = {"policies": {}, "outputs": {}}
+    rng = np.random.default_rng(5)
+    for pol, s, n in LIVE_POLICY_RUNS:
+        ref_pol = getattr(archive, pol)()
+        live["policies"][pol] = sha_policy(ref_pol)
+        digests = []
+        for i in range(n):
+            img = live_input(rng, s, i)
+            random.seed(i)
+            np.random.seed(i)
+            policy = random.choice(ref_pol)
+            im = PIL.Image.fromarray(img)
+            for name, pr, level in policy:
+                if random.random() > pr:
+                    continue
+                im = aug.apply_augment(im, name, level)
+            digests.append(sha(np.asarray(im))[:16])
+        live["outputs"]["%s_%d" % (pol, s)] = digests
+    hashes["live_reference"] = live
+
+    # ---- (8) ToTensor -> Lighting(0.1, PCA) -> Normalize of the ImageNet train chain (data.py:70-72), fp32, per image
+    lighting = T.Compose([T.ToTensor(), aug.Lighting(0.1, data._IMAGENET_PCA["eigval"], data._IMAGENET_PCA["eigvec"]),
+                          T.Normalize(mean=[0.485, 0.456, 0.406], std=[0.229, 0.224, 0.225])])
+    batch = synth_batch(40, (64, 72), seed=4)
+    torch.manual_seed(5)
+    hashes["lighting_chain"] = [sha(lighting(PIL.Image.fromarray(a)).numpy())[:16] for a in batch]
 
     np.savez_compressed(os.path.join(HERE, "golden_chain.npz"), **chain)
     with open(os.path.join(HERE, "golden_hashes.json"), "w") as f:

@@ -33,6 +33,56 @@ def synth_batch(n, shape, seed):
     return np.stack([synth(shape, i % 3, rng) for i in range(n)])
 
 
+# (policy, image shape, batch) of the policy-level fixtures of tests/golden/golden_chain.npz, drawn in this order
+GOLDEN_POLICY_BATCHES = (("fa_reduced_cifar10", (32, 32), 96), ("autoaug_policy", (32, 32), 96),
+                         ("fa_reduced_svhn", (32, 32), 48), ("arsaug_policy", (24, 40), 48),
+                         ("fa_resnet50_rimagenet", (56, 56), 48))
+
+
+def make_chain_inputs():
+    """The seeded inputs that tests/golden/make_golden.py feeds to the reference for golden_chain.npz."""
+    rng = np.random.default_rng(77)
+    ins = {}
+    for pol, shape, n in GOLDEN_POLICY_BATCHES:
+        ins["policy_%s_in" % pol] = np.stack([synth(shape, i % 3, rng) for i in range(n)])
+    rng = np.random.default_rng(99)
+    ins["cifar_chain_in"] = np.stack([synth((32, 32), i % 3, rng) for i in range(64)])
+    return ins
+
+
+# (policy, image size, images) of the whole-policy digests in golden_hashes.json["live_reference"], drawn in this order
+LIVE_POLICY_RUNS = (("fa_reduced_cifar10", 32, 400), ("autoaug_policy", 32, 400), ("fa_resnet50_rimagenet", 64, 100))
+
+
+def live_input(rng, s, i):
+    """Image i of a whole-policy run: noise for odd i, a low-contrast ramp for even i."""
+    if i % 2:
+        return rng.integers(0, 256, (s, s, 3), dtype=np.uint8)
+    return np.clip(np.linspace(60, 180, s)[None, :, None] + rng.normal(0, 6, (s, s, 3)), 0, 255).astype(np.uint8)
+
+
+def sha_policy(policies):
+    """Digest of a policy table, [[(name, prob, level), ...], ...]: equal digests <=> equal tables under `==`."""
+    import hashlib
+    import json
+    rows = [[[str(name), float(p), float(lvl)] for name, p, lvl in sub] for sub in policies]
+    return hashlib.sha256(json.dumps(rows).encode()).hexdigest()
+
+
+def golden_chain():
+    """golden_chain.npz (the reference's outputs) plus the inputs they were computed from; the regenerated inputs
+    must match the digests make_golden.py recorded, so a change in NumPy's generators cannot pass unnoticed."""
+    import hashlib
+    import json
+    with open(os.path.join(GOLDEN, "golden_hashes.json")) as f:
+        want = json.load(f)["chain_inputs"]
+    g = dict(np.load(os.path.join(GOLDEN, "golden_chain.npz")))
+    for k, a in make_chain_inputs().items():
+        assert hashlib.sha256(a.tobytes()).hexdigest() == want[k], k
+        g[k] = a
+    return g
+
+
 def exact_norm_table(mean, std):
     """fp32 ToTensor+Normalize value of every byte, computed with torch itself."""
     import torch

@@ -6,7 +6,6 @@ pixel evaluation from tests/emu - and demand bit-exact agreement with the oracle
 (oracle.pil_path = the reference's calls into Pillow) on every op, policy and chain.
 """
 import json
-import os
 import random
 
 import numpy as np
@@ -14,7 +13,7 @@ import PIL.Image
 import pytest
 import torch
 
-from helpers import ALL_OPS, GOLDEN, emu_augment, exact_norm_table, seed_all, synth_batch
+from helpers import ALL_OPS, emu_augment, exact_norm_table, golden_chain, seed_all, synth_batch
 
 from fast_autoaugment_b200 import archive
 from fast_autoaugment_b200.engine import CIFAR_MEAN, CIFAR_STD, IMAGENET_MEAN, IMAGENET_STD, CompiledPolicy, TailSpec
@@ -98,7 +97,7 @@ def test_all_op_pairs(emu):
 def test_cifar_chain_fp32_matches_golden_and_oracle(emu):
     """Augmentation -> RandomCrop(32,4) -> HFlip -> ToTensor -> Normalize -> CutoutDefault(16):
     the exact transform_train of reference data.py:39-44,92,112, fp32, max abs diff 0."""
-    g = np.load(os.path.join(GOLDEN, "golden_chain.npz"))
+    g = golden_chain()
     batch, want = g["cifar_chain_in"], g["cifar_chain_out_f32"]
     policies = archive.fa_reduced_cifar10()
     pol = CompiledPolicy(policies)

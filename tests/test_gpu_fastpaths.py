@@ -7,6 +7,8 @@ twice: forced through the two-kernel split (FAA_SPLIT_MIN=0) and forced through 
 fp32 output must be bit-exact (exact ToTensor+Normalize table of the oracle's uint8 result); fp16 / bf16 must
 equal that fp32 value rounded once.
 """
+import hashlib
+import json
 import os
 import random
 
@@ -15,7 +17,7 @@ import PIL.Image
 import pytest
 import torch
 
-from helpers import ALL_OPS, exact_norm_table, seed_all, synth_batch
+from helpers import ALL_OPS, GOLDEN, exact_norm_table, seed_all, synth_batch
 
 from fast_autoaugment_b200 import _lib
 from fast_autoaugment_b200.engine import IMAGENET_MEAN, IMAGENET_STD, CIFAR_MEAN, CIFAR_STD, CompiledPolicy, TailSpec, augment_batch
@@ -175,21 +177,14 @@ def test_color_jitter_matches_torchvision():
 
 def test_lighting_folded_into_the_normalisation_matches_the_reference_chain():
     """row N2: ToTensor -> Lighting(0.1, PCA) -> Normalize (reference data.py:70-72, augmentations.py:197-215) as
-    per-image normalisation tables; the reference's own Lighting class (oracle/_ref) or its restatement is the oracle"""
-    from torchvision import transforms
-    from fast_autoaugment_b200.data import Lighting, _IMAGENET_PCA
-    try:
-        from oracle import build_ref
-        mods = build_ref.import_ref()
-        RefLighting = mods[0].Lighting if mods is not None else Lighting
-    except Exception:
-        RefLighting = Lighting
+    per-image normalisation tables; the oracle is the reference's own chain, recorded image by image by
+    tests/golden/make_golden.py (torch.manual_seed(5), the same inputs)"""
+    from fast_autoaugment_b200.data import Lighting
+    with open(os.path.join(GOLDEN, "golden_hashes.json")) as f:
+        want = json.load(f)["lighting_chain"]
     n, shape = 40, (64, 72)
     batch = synth_batch(n, shape, seed=4)
-    ref_chain = transforms.Compose([transforms.ToTensor(), RefLighting(0.1, _IMAGENET_PCA["eigval"], _IMAGENET_PCA["eigvec"]),
-                                    transforms.Normalize(mean=IMAGENET_MEAN, std=IMAGENET_STD)])
-    torch.manual_seed(5)
-    want = torch.stack([ref_chain(PIL.Image.fromarray(a)) for a in batch])
+    assert len(want) == n
     torch.manual_seed(5)
     rgb = Lighting(0.1).sample_rgb(n)
     pol = CompiledPolicy([[("Invert", 0.0, 0.0), ("Invert", 0.0, 0.0)]])
@@ -199,7 +194,8 @@ def test_lighting_folded_into_the_normalisation_matches_the_reference_chain():
     for split in ("0", "1000000000000"):
         os.environ["FAA_SPLIT_MIN"] = split
         got = augment_batch(pol, x, TailSpec(None, 0, False, IMAGENET_MEAN, IMAGENET_STD, 0, torch.float32), z, zb, lighting_rgb=rgb).cpu()
-        assert torch.equal(got, want), split
+        bad = [i for i in range(n) if hashlib.sha256(got[i].numpy().tobytes()).hexdigest()[:16] != want[i]]
+        assert got.dtype == torch.float32 and got.shape == (n, 3) + shape and not bad, (split, bad)
     os.environ.pop("FAA_SPLIT_MIN", None)
     # with a policy in front and a flip behind it: equals the un-lit launch re-normalised image by image
     pol2 = CompiledPolicy([[("Rotate", 1.0, 0.3), ("Color", 1.0, 0.6)], [("AutoContrast", 1.0, 0.3), ("Sharpness", 1.0, 0.8)]])

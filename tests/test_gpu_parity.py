@@ -5,7 +5,6 @@ fp32 oracle rounded to that dtype.  Full-size cases (BASELINE.json configs) are 
 through the host emulation of the same source, through size-independent properties, and
 against the oracle on a sample of the batch.
 """
-import os
 import random
 
 import numpy as np
@@ -13,7 +12,7 @@ import PIL.Image
 import pytest
 import torch
 
-from helpers import ALL_OPS, GOLDEN, emu_augment, exact_norm_table, seed_all, synth_batch
+from helpers import ALL_OPS, emu_augment, exact_norm_table, golden_chain, seed_all, synth_batch
 
 from fast_autoaugment_b200 import _lib, archive
 from fast_autoaugment_b200.engine import (CIFAR_MEAN, CIFAR_STD, IMAGENET_MEAN, IMAGENET_STD, CompiledPolicy,
@@ -103,7 +102,7 @@ def test_archive_policies(pol_name, shape, n):
 
 def test_golden_policy_outputs():
     """committed outputs of the live reference (tests/golden/make_golden.py)"""
-    g = np.load(os.path.join(GOLDEN, "golden_chain.npz"))
+    g = golden_chain()
     for pol_name in ("fa_reduced_cifar10", "autoaug_policy", "fa_reduced_svhn", "arsaug_policy",
                      "fa_resnet50_rimagenet"):
         batch, want = g["policy_%s_in" % pol_name], g["policy_%s_out" % pol_name]
@@ -117,7 +116,7 @@ def test_golden_policy_outputs():
 def test_golden_cifar_chain_all_dtypes():
     """transform_train of reference data.py:39-44,92,112: fp32 bit-exact; fp16/bf16 equal the
     fp32 result rounded to that dtype (uint8-level parity is implied, SURVEY.md 8c-12)"""
-    g = np.load(os.path.join(GOLDEN, "golden_chain.npz"))
+    g = golden_chain()
     batch, want = g["cifar_chain_in"], torch.from_numpy(g["cifar_chain_out_f32"])
     pol = CompiledPolicy(archive.fa_reduced_cifar10())
     for dt in (torch.float32, torch.float16, torch.bfloat16):
