@@ -745,9 +745,12 @@ static int augment_common(faa_policy_t* p, const uint8_t* d_in_all, int n_all, i
     // program slots by completion counters the next resolve kernel of the slot waits for, scratch images by a copy per slot.
     static const bool persist_off = [] { const char* e = getenv("FAA_PERSIST"); return e && e[0] == '0'; }();
     const bool persist = use_chain && !persist_off;
-    size_t scratch_slot_bytes = 0;
+    // The copy of slot 1 starts at a fixed half of the allocation, not behind this call's n_all images: the resolve kernel of
+    // a slot only waits for that slot's previous readers, so after a batch-size change a slot's scratch must not move onto
+    // the images the other slot's step - two steps back, possibly still running - reads.
+    size_t scratch_half = 0;
     if ((p->has_sg || use_mid) && !d_partner && (w & 3) == 0) {
-        scratch_slot_bytes = (size_t)n_all * img_bytes;
+        const size_t scratch_slot_bytes = ((size_t)n_all * img_bytes + 255) & ~(size_t)255;
         const size_t need = scratch_slot_bytes * (persist ? 2 : 1);
         if (p->d_scratch_bytes < need) {
             if (p->d_scratch) { CK(cudaStreamSynchronize(stream)); CK(cudaFree(p->d_scratch)); p->d_scratch = nullptr; p->d_scratch_bytes = 0; }
@@ -755,6 +758,7 @@ static int augment_common(faa_policy_t* p, const uint8_t* d_in_all, int n_all, i
             p->d_scratch_bytes = need;
         }
         P.scratch = (uint8_t*)p->d_scratch;
+        scratch_half = (p->d_scratch_bytes / 2) & ~(size_t)255;      // >= scratch_slot_bytes whenever persist
         R.allow |= 2;
     }
     // With the lean gathers (allow bit 2) and a scratch image (bit 1) every program of a three-way split is light or mid
@@ -896,7 +900,7 @@ static int augment_common(faa_policy_t* p, const uint8_t* d_in_all, int n_all, i
         if (persist) {
             if (!p->sm_count) CK(cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, p->device));
             Pc.done = done_word(slot);
-            if (P.scratch) Pc.scratch = P.scratch + (size_t)slot * scratch_slot_bytes;
+            if (P.scratch) Pc.scratch = P.scratch + (size_t)slot * scratch_half;
         }
         AugParams Pm = Pc;                                  // the mid kernel: its own (taller) bands in bands / geo[0]
         if (use_mid) set_mid_geometry(Pm);

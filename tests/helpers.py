@@ -93,6 +93,28 @@ def exact_norm_table(mean, std):
     return ((x[None, :] - m) / s).numpy().astype(np.float32).copy()
 
 
+# mean / std for which a fused multiply-add does NOT round like torch's (u / 255 - mean) / std in that dtype: the
+# half-precision launches take the exact normalisation table (the TAB=true light / mid / cluster kernels)
+TABLE_STATS = {"float16": ((0.7838, 0.3033, 0.4766), (0.2959, 0.455, 0.2573)),
+               "bfloat16": ((0.2401, 0.9531, 0.3522), (0.1511, 0.186, 0.474))}
+
+
+def fma_shortcut_rounds_like_the_table(mean, std, dt):
+    """The host's rule (faa_cabi.cu normalisation()): for every channel and byte u, the dt-rounded
+    fmaf(u, (float)(1 / (255 std)), (float)(-mean / std)) equals the dt-rounded exact value.  u * scale + bias is exact in
+    float64 at these magnitudes (a 32-bit product plus a 24-bit addend within 2^4), so one rounding to float32 is fmaf."""
+    import torch
+    tab = torch.from_numpy(exact_norm_table(mean, std))
+    u = np.arange(256, dtype=np.float64)
+    for c in range(3):
+        s, m = float(np.float32(std[c])), float(np.float32(mean[c]))
+        scale, bias = float(np.float32(1.0 / (255.0 * s))), float(np.float32(-m / s))
+        fma = torch.from_numpy((u * scale + bias).astype(np.float32))
+        if not torch.equal(fma.to(dt), tab[c].to(dt)):
+            return False
+    return True
+
+
 def emu_augment(emu, pol, batch_u8, samples, boxes, tail=None, norm=None, partner=None, lam=1.0,
                 force_generic=False, pool=None, pool_samples=None, pool_boxes=None, first=0):
     """Drive tests/emu like engine.augment_batch drives the kernels.  norm=None -> uint8 HWC."""

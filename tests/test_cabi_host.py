@@ -380,3 +380,15 @@ def test_ragged_sub_policies_replay_the_reference_draws():
     seed_all(6)
     c, cb, _, _ = pol.sample_policy_mt(200, 32, 32)
     assert a[["sub", "gate", "sign"]].tobytes() == c[["sub", "gate", "sign"]].tobytes() and ab.tobytes() == cb.tobytes()
+
+
+def test_fma_normalisation_shortcut_rule():
+    """The rule the host applies before a half-precision launch takes the fma shortcut instead of the exact table
+    (faa_cabi.cu normalisation()): the shipped CIFAR / ImageNet stats pass it in fp16 and bf16, the custom stats of the
+    exact-table GPU tests fail it in their dtype - if either changed, those tests would silently run the other kernels."""
+    from helpers import TABLE_STATS, fma_shortcut_rounds_like_the_table
+    for mean, std in ((engine.CIFAR_MEAN, engine.CIFAR_STD), (engine.IMAGENET_MEAN, engine.IMAGENET_STD)):
+        for dt in (torch.float16, torch.bfloat16):
+            assert fma_shortcut_rounds_like_the_table(mean, std, dt)
+    for name, (mean, std) in TABLE_STATS.items():
+        assert not fma_shortcut_rounds_like_the_table(mean, std, getattr(torch, name))

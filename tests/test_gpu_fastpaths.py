@@ -17,7 +17,7 @@ import PIL.Image
 import pytest
 import torch
 
-from helpers import ALL_OPS, GOLDEN, exact_norm_table, seed_all, synth_batch
+from helpers import ALL_OPS, GOLDEN, TABLE_STATS, exact_norm_table, fma_shortcut_rounds_like_the_table, seed_all, synth_batch
 
 from fast_autoaugment_b200 import _lib
 from fast_autoaugment_b200.engine import IMAGENET_MEAN, IMAGENET_STD, CIFAR_MEAN, CIFAR_STD, CompiledPolicy, TailSpec, augment_batch
@@ -56,15 +56,20 @@ def _policies():
 
 
 @pytest.mark.parametrize("split_min", ["0", "1000000000000"])
-@pytest.mark.parametrize("shape,norm", [((48, 64), "imagenet"), ((224, 224), "imagenet"), ((56, 104), "cifar"), ((380, 376), "imagenet")])
+@pytest.mark.parametrize("shape,norm", [((48, 64), "imagenet"), ((224, 224), "imagenet"), ((56, 104), "cifar"), ((380, 376), "imagenet"),
+                                        ((224, 224), "float16"), ((56, 104), "bfloat16")])
 def test_octet_paths_match_oracle(shape, norm, split_min, monkeypatch):
+    """norm "float16" / "bfloat16": Normalize stats for which the fma shortcut does not round like the exact table in that
+    dtype, so its launches run the TAB=true light / mid (split) or cluster kernels"""
     monkeypatch.setenv("FAA_SPLIT_MIN", split_min)
     H, W = shape
     policies = _policies()
     n = len(policies)
     pol = CompiledPolicy(policies)
     batch = synth_batch(n, shape, seed=H * 3 + W)
-    mean, std = (IMAGENET_MEAN, IMAGENET_STD) if norm == "imagenet" else (CIFAR_MEAN, CIFAR_STD)
+    mean, std = {"imagenet": (IMAGENET_MEAN, IMAGENET_STD), "cifar": (CIFAR_MEAN, CIFAR_STD)}.get(norm) or TABLE_STATS[norm]
+    if norm in TABLE_STATS:
+        assert not fma_shortcut_rounds_like_the_table(mean, std, getattr(torch, norm))
     seed_all(4)
     want_u8 = np.stack([np.asarray(pil_path.PolicyTransform([policies[i]])(PIL.Image.fromarray(a)))
                         for i, a in enumerate(batch)])
@@ -196,6 +201,9 @@ def test_lighting_folded_into_the_normalisation_matches_the_reference_chain():
         got = augment_batch(pol, x, TailSpec(None, 0, False, IMAGENET_MEAN, IMAGENET_STD, 0, torch.float32), z, zb, lighting_rgb=rgb).cpu()
         bad = [i for i in range(n) if hashlib.sha256(got[i].numpy().tobytes()).hexdigest()[:16] != want[i]]
         assert got.dtype == torch.float32 and got.shape == (n, 3) + shape and not bad, (split, bad)
+        for dt in (torch.float16, torch.bfloat16):          # the per-image tables, then ONE rounding at the store
+            half = augment_batch(pol, x, TailSpec(None, 0, False, IMAGENET_MEAN, IMAGENET_STD, 0, dt), z, zb, lighting_rgb=rgb).cpu()
+            assert half.dtype == dt and torch.equal(half, got.to(dt)), (split, dt)
     os.environ.pop("FAA_SPLIT_MIN", None)
     # with a policy in front and a flip behind it: equals the un-lit launch re-normalised image by image
     pol2 = CompiledPolicy([[("Rotate", 1.0, 0.3), ("Color", 1.0, 0.6)], [("AutoContrast", 1.0, 0.3), ("Sharpness", 1.0, 0.8)]])
@@ -208,6 +216,10 @@ def test_lighting_folded_into_the_normalisation_matches_the_reference_chain():
         t = u8[i].permute(2, 0, 1).float().div(255)
         t = t.add(rgb[i].view(3, 1, 1).expand_as(t))
         assert torch.equal(lit[i], (t - m) / sd), i
+    for dt in (torch.float16, torch.bfloat16):
+        half = augment_batch(pol2, x, TailSpec.imagenet(0, dt), s2, b2, lighting_rgb=rgb).cpu()
+        bad = [i for i in range(n) if not torch.equal(half[i], lit[i].to(dt))]
+        assert not bad, (dt, bad)
 
 
 @pytest.mark.gpu
